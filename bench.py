@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the VITS inference hot path (BASELINE.json metric: audio-seconds/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One JSON line on rank 0's stdout (contract in the task statement; DESIGN.md "Measurement").
@@ -20,6 +20,10 @@ rank 0 over NCCL INSIDE the timed region (the "trivial batch scatter/gather" of 
 `--impl reference` times the reference's own CPU implementation of the path on the host cores: the unmodified
 `SynthesizerTrn.infer` from oracle/_ref (placed by oracle/build_ref.py; kind "reference") when present, else the oracle
 port (kind "port"), on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step returned (waveforms, and the valid frame counts where the step
+returns them) to DIR/<name>.npy, at most 64 MB in all, so that two builds can be compared output for output: the inputs
+are seeded, so the same arguments give the same inputs on every run.
 """
 import argparse
 import contextlib
@@ -49,6 +53,7 @@ import torch  # noqa: E402
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 CLI_TOKENS = "sil j in1 #0 t ian1 #0 t ian1 #0 q i4 #0 z en3 #0 m e5 #0 ^ iang4 #4".split()   # SURVEY.md 8(d) config 1
 CLI_VOCAB = ["sil"] + sorted(set(CLI_TOKENS) - {"sil"})
@@ -95,6 +100,35 @@ def make_batch(wl, B, seed):
     lens = torch.full((B,), x.shape[1], dtype=torch.long)
     sid = torch.randint(0, wl["n_spk"], (B,), generator=gen)
     return x, lens, sid
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(arrays, out_dir):
+    """Writes `arrays` (name -> tensor) as out_dir/<name>.npy: floating point as float32 (float64 stays float64),
+    integers as float64 (exact).  Arrays up to 1 MiB are written whole; when the larger ones exceed the rest of
+    DUMP_BYTES together, each keeps a share of rows (first dimension, one utterance each) proportional to its size: a
+    sorted sample drawn with a fixed seed, so it depends on the shapes only, and the indices of the kept rows go to
+    out_dir/<name>_rows.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().cpu() for k, v in arrays.items()}
+    host = {k: v.double() if not v.is_floating_point() or v.dtype == torch.float64 else v.float() for k, v in host.items()}
+    size = {k: v.numel() * v.element_size() for k, v in host.items()}
+    large = {k for k, n in size.items() if n > 1 << 20}
+    total = sum(size[k] for k in large)
+    budget = DUMP_BYTES - sum(n for k, n in size.items() if k not in large) - 4096 * 2 * len(host)   # .npy headers
+    for name, v in host.items():
+        nbytes = size[name]
+        if name in large and total > budget and v.shape[0] > 1:
+            row_bytes = nbytes // v.shape[0] + 8                # + its index in <name>_rows.npy
+            keep = max(1, min(v.shape[0], int(budget * nbytes / total) // row_bytes))
+            if keep < v.shape[0]:
+                rows = torch.randperm(v.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+                np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.double().numpy())
+                v = v[rows]
+        np.save(os.path.join(out_dir, f"{name}.npy"), v.contiguous().numpy())
 
 
 class ClockSampler:
@@ -194,8 +228,7 @@ class CpuArm:
         self.sd = synth.make_state_dict(self.hps.model, self.wl["n_vocab"], self.wl["n_spk"], seed=self.hps.train.seed)
         self.kind, self.net, self.w = "port", None, None
         try:
-            from oracle import build_ref, ref_harness
-            build_ref.build()
+            from oracle import ref_harness
             if ref_harness.available():
                 with contextlib.redirect_stdout(io.StringIO()):
                     self.net = ref_harness.build_reference_model(self.hps, self.wl["n_vocab"], self.wl["n_spk"], self.sd)
@@ -496,7 +529,8 @@ def run_ours(args):
     def timed(fn, steps, drain=None):
         """EXACTLY `steps` steps between barrier + synchronize; device time from CUDA events on the launch stream
         (per step, so an L2 flush between steps stays outside); `drain` (pipelined copies) runs before the closing event,
-        which is recorded after the launch stream has waited for the last copy; returns (max over ranks, this rank's) ms."""
+        which is recorded after the launch stream has waited for the last copy; returns (max over ranks, this rank's) ms
+        and what the last step returned."""
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         ev_end = torch.cuda.Event(enable_timing=True)
         barrier()
@@ -504,8 +538,10 @@ def run_ours(args):
             if flush_buf is not None:
                 flush_buf.fill_(i & 0xFF)
             ev[i][0].record()
-            fn()
+            out = fn()
             ev[i][1].record()
+            if i + 1 < steps:
+                out = None      # released before the next step, as if never held: its memory is reused there
         if drain is not None:
             drain()
         ev_end.record()
@@ -514,7 +550,7 @@ def run_ours(args):
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
         if dist:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item()), ms
+        return float(t.item()), ms, out
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
@@ -523,11 +559,22 @@ def run_ours(args):
     sampler.start()
     if args.profile_range:
         torch.cuda.profiler.start()
-    total_ms, my_ms = timed(step_resident, args.steps)
+    total_ms, my_ms, last = timed(step_resident, args.steps)
     if args.profile_range:
         torch.cuda.profiler.stop()
     clocks = sampler.stop()
     launches = net.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        if kind == "generator":
+            outs = {"audio": last}
+        elif sharded:
+            outs = {"audio": last[0], "audio_index_and_samples": last[1]}
+        else:
+            outs = {"audio" if len(last) == 1 else f"audio_{i}": o_ for i, o_ in enumerate(last)}
+            if chunk is None:
+                outs["y_lengths"] = net.last_y_lengths
+        dump_outputs(outs, args.dump_outputs)
+    last = None
 
     if kind != "generator":
         frames_rank = state.get("frames_local", state["frames"]) if sharded else state["frames"]
@@ -537,7 +584,7 @@ def run_ours(args):
     for _ in range(2):
         step_e2e()
     d2h_drain()
-    e2e_ms, _ = timed(step_e2e, args.steps, drain=d2h_drain)
+    e2e_ms, _, _ = timed(step_e2e, args.steps, drain=d2h_drain)
     if kind != "generator":
         d2h = state["d2h"] + 8
 
@@ -684,7 +731,12 @@ def main():
                     help="operand format of the fused stage kernels: 16 = f16 split, 32 = 3xTF32, 0 = library default")
     ap.add_argument("--attention-tc", type=int, default=-1, help="1/0: text-encoder attention on the tensor pipe (-1: library default)")
     ap.add_argument("--length-aware", type=int, default=0, help="1: skip generator tiles beyond each utterance's own length")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/<name>.npy (rank 0; at most 64 MB, rows sampled "
+                         "with a fixed seed beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,6 +1,7 @@
-"""Generate tests/golden/*.npz by running the REAL reference (authoring container only).
+"""Generate tests/golden/*.npz and tests/golden/reference_state_dict_layout.json by running the REAL reference
+(needs a checkout of wetts; see oracle/ref_harness.py).
 
-    python -m oracle.gen_golden            # from the repo root
+    python -m oracle.gen_golden [NAME ...]            # from the repo root; NAME = a case or the layout file
 
 For each case: build the seeded synthetic checkpoint (wetts_b200/synth.py), load it into
 the reference's own SynthesizerTrn (`/root/reference/wetts/vits/model/models.py`), run
@@ -8,6 +9,7 @@ the reference's own SynthesizerTrn (`/root/reference/wetts/vits/model/models.py`
 The fixtures pin oracle/vits_oracle.py (tests/test_oracle_golden.py) and are the final
 arbiter for the CUDA path (tests/test_parity_gpu.py).  Test infrastructure only.
 """
+import json
 import os
 import sys
 
@@ -44,6 +46,25 @@ CASES = [
 CLI_TOKENS = "sil j in1 #0 t ian1 #0 t ian1 #0 q i4 #0 z en3 #0 m e5 #0 ^ iang4 #4".split()
 CLI_VOCAB = ["sil"] + sorted(set(CLI_TOKENS) - {"sil"})
 
+# state-dict layout (name -> shape) of the reference's SynthesizerTrn, which tests/test_host_cpu.py checks the synthetic
+# checkpoint against: config, n_vocab, n_speakers
+LAYOUT_CASES = [("multilingual_v3", 40, 2), ("baker_v1", 40, 2)]
+LAYOUT_FILE = "reference_state_dict_layout.json"
+
+
+def write_state_dict_layout():
+    out = {}
+    for cfg_name, n_vocab, n_spk in LAYOUT_CASES:
+        hps = builtin_config(cfg_name)
+        net = ref_harness.build_reference_model(hps, n_vocab, n_spk, synth.make_state_dict(hps.model, n_vocab, n_spk, seed=3))
+        out[cfg_name] = {"n_vocab": n_vocab, "n_speakers": n_spk,
+                         "state_dict": {k: list(v.shape) for k, v in net.state_dict().items()}}
+    path = os.path.join(GOLDEN_DIR, LAYOUT_FILE)
+    with open(path, "w") as f:
+        json.dump(out, f, indent=0, sort_keys=True)
+        f.write("\n")
+    print(LAYOUT_FILE, {k: len(v["state_dict"]) for k, v in out.items()}, os.path.getsize(path) // 1024, "KiB")
+
 
 def make_inputs(n_vocab, n_speakers, x_lengths, seed, max_frames_per_phone=40):
     gen = torch.Generator().manual_seed(seed)
@@ -61,6 +82,8 @@ def main():
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     torch.set_num_threads(1)
     only = set(sys.argv[1:])
+    if not only or LAYOUT_FILE in only:
+        write_state_dict_layout()
     for name, cfg_name, n_vocab, n_spk, x_lengths, scales, seed in CASES:
         if only and name not in only:
             continue

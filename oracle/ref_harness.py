@@ -17,10 +17,10 @@ import types
 import torch
 
 REFERENCE_ROOT = "/root/reference"
-# the reference tree where it lies (authoring container) or the byte-identical copy placed by oracle/build_ref.py
-# under oracle/_ref/ (git-ignored; travels to the GPU box)
-_CANDIDATES = (os.path.join(REFERENCE_ROOT, "wetts", "vits"),
-               os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref", "wetts_vits"))
+# the byte-identical copy that oracle/build_ref.py places under oracle/_ref/ (git-ignored) when the build ran next to a
+# wetts checkout, else that checkout itself
+_CANDIDATES = (os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref", "wetts_vits"),
+               os.path.join(REFERENCE_ROOT, "wetts", "vits"))
 _VITS_DIR = next((d for d in _CANDIDATES if os.path.isfile(os.path.join(d, "model", "models.py"))), _CANDIDATES[0])
 
 

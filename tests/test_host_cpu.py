@@ -1,5 +1,6 @@
 """CPU-side checks: the C-ABI library loads and exports every declared symbol, host logic
 (config mirror, synthetic checkpoints, loud failure without a GPU)."""
+import json
 import os
 import re
 
@@ -81,15 +82,21 @@ def test_vits2_vocos_recipe_constructs_and_maps_its_config():
 
 
 def test_reference_loads_synthetic_checkpoint():
-    """Where the reference tree exists (authoring container) the synthetic state dict must load
-    into the reference's own module with nothing unexpected and only enc_q.* missing."""
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference tree not present")
-    for cfg in ("multilingual_v3", "baker_v1"):
+    """The synthetic state dict must load into the reference's own module: against the reference's state-dict layout
+    (name -> shape, recorded by oracle/gen_golden.py), nothing unexpected, no shape mismatch, and the only missing
+    tensors are the ones infer never reads (posterior encoder, iSTFT window, VITS2 post_transformer)."""
+    layout = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_state_dict_layout.json")))
+    assert set(layout) == {"multilingual_v3", "baker_v1"}
+
+    def unused(k):
+        return k.startswith("enc_q.") or k.startswith("dec.istft.") or ".post_transformer." in k
+    for cfg, spec in layout.items():
         hps = builtin_config(cfg)
-        sd = synth.make_state_dict(hps.model, 40, 2, seed=3)
-        ref_harness.build_reference_model(hps, 40, 2, sd)
+        sd = synth.make_state_dict(hps.model, spec["n_vocab"], spec["n_speakers"], seed=3)
+        ref = spec["state_dict"]
+        assert [k for k in sd if k not in ref] == [], cfg
+        assert [k for k in sd if list(sd[k].shape) != ref[k]] == [], cfg
+        assert [k for k in ref if k not in sd and not unused(k)] == [], cfg
 
 
 def test_mma_issue_paths_stay_in_the_uniform_datapath():
