@@ -100,11 +100,15 @@ int wetts_vits_create(const wetts_vits_config* cfg, int device, wetts_vits_t* ou
  * (e.g. "dec.ups.0.weight_v"; key patterns: SURVEY.md App. B).  fp32, contiguous,
  * host or device memory; the engine keeps its own device copy.  Accepts both
  * weight-normed pairs (`weight_g`/`weight_v`, what inference.py loads) and folded
- * `weight` (what export_onnx.py:79-81 produces).  `enc_q.*` keys are ignored. */
+ * `weight` (what export_onnx.py:79-81 produces).  `enc_q.*` keys (the posterior encoder) are
+ * kept for voice conversion; infer never reads them. */
 int wetts_vits_set_tensor(wetts_vits_t h, const char* name, const void* data, const int64_t* dims, int ndim);
 /* Fold weight-norm (per out-channel for Conv1d, per IN-channel for ConvTranspose1d,
  * decoders.py:41-48) and re-lay weights for the kernels.  Fails listing the first
- * missing key.  Synchronous. */
+ * missing key.  The posterior encoder (enc_q.*) is packed only when every one of its
+ * keys is present; a checkpoint without it, or with an incomplete one, finalizes all
+ * the same and the voice-conversion calls below then fail naming the first missing
+ * key.  Synchronous. */
 int wetts_vits_finalize(wetts_vits_t h);
 void wetts_vits_destroy(wetts_vits_t h);
 /* Per-handle options; they take precedence over the process-wide ones above.  "tensor_cores" and
@@ -162,6 +166,12 @@ size_t wetts_flow_workspace_bytes(wetts_vits_t h, int B, int Ty);
 int wetts_flow_reverse(wetts_vits_t h, float* z, const int64_t* y_lengths, const float* g, int B, int Ty,
                        void* workspace, size_t workspace_bytes, void* stream);
 
+/* ResidualCouplingTransformersBlock.forward(reverse=False): the four coupling layers in
+ * forward order, x1 = m + x1 * mask (flows.py:494-513).  z f32[B,192,Ty] IN PLACE (z -> z_p);
+ * workspace sized by wetts_flow_workspace_bytes. */
+int wetts_flow_forward(wetts_vits_t h, float* z, const int64_t* y_lengths, const float* g, int B, int Ty,
+                       void* workspace, size_t workspace_bytes, void* stream);
+
 /* Generator.forward (decoders.py:63-82): z f32[B,192,T] (+ g f32[B,gin] or NULL)
  * -> audio f32[B,1,T*U].  If y_lengths != NULL the input is multiplied by the frame
  * mask first, as infer() does (models.py:271). */
@@ -197,6 +207,41 @@ int wetts_vits_infer_synthesize(wetts_vits_t h, const int64_t* x_lengths, const 
                                 const float* scales3, const float* noise_z, int64_t noise_bs, int64_t noise_rs,
                                 int B, int Tx, int Ty, int gen_frames, float* audio, float* attn, float* y_mask, float* z,
                                 float* z_p, float* m_p, float* logs_p, void* workspace, size_t workspace_bytes,
+                                void* stream);
+
+/* ---- voice conversion (SynthesizerTrn.voice_conversion, models.py:369-376) ----------------
+ * Need a checkpoint with the complete posterior encoder (enc_q.*). */
+
+/* PosteriorEncoder.forward (encoders.py:91-99): y f32[B,S,T] features (S = the in-channels of
+ * enc_q.pre: filter_length/2+1 linear bins, or n_mel_channels for a VITS2 mel posterior),
+ * y_lengths int64[B], g f32[B,gin] or NULL, noise f32[B,192,T] explicit N(0,1) draws (required,
+ * what the reference draws with randn_like) -> z f32[B,192,T]; m, logs f32[B,192,T] may be NULL. */
+size_t wetts_posterior_workspace_bytes(wetts_vits_t h, int B, int T);
+int wetts_posterior_encoder_forward(wetts_vits_t h, const float* y, const int64_t* y_lengths, const float* g,
+                                    const float* noise, int B, int T, float* z, float* m, float* logs,
+                                    void* workspace, size_t workspace_bytes, void* stream);
+
+/* Linear spectrogram, spectrogram_torch(center=False) (mel_processing.py:42-93) applied to each
+ * utterance on its own: reflection padding by p = (n_fft - hop)/2 at the utterance's own length,
+ * periodic Hann window, onesided real DFT, sqrt(re^2 + im^2 + 1e-6).  n_fft = win = 2 (S - 1)
+ * (S - 1 a power of two), hop = wetts_vits_upsample_factor.  audio f32[B,L], audio_lengths
+ * int64[B] (each in [p+1, L]) -> spec f32[B,S,F] with F = 1 + (L + 2p - n_fft)/hop, frames at or
+ * beyond an utterance's own count F_b = 1 + (L_b + 2p - n_fft)/hop exactly 0; spec_lengths
+ * int64[B] = F_b (may be NULL).  Checks the lengths on the host: synchronises `stream`.
+ * The workspace query returns 0 when L is too short or the model has no spectrogram. */
+size_t wetts_spectrogram_workspace_bytes(wetts_vits_t h, int B, int64_t L);
+int wetts_spectrogram(wetts_vits_t h, const float* audio, const int64_t* audio_lengths, int B, int64_t L, float* spec,
+                      int64_t* spec_lengths, void* workspace, size_t workspace_bytes, void* stream);
+
+/* The whole conversion: posterior encoder and forward flow with g = emb_g(sid_src), inverse flow
+ * and generator with g = emb_g(sid_tgt) on z_hat * y_mask over all T frames.  y / y_lengths /
+ * noise as for wetts_posterior_encoder_forward; sid_src, sid_tgt int64[B].  Outputs (any may be
+ * NULL except audio): audio f32[B,1,T*U], y_mask f32[B,1,T], z, z_p, z_hat f32[B,192,T].
+ * Fails for a single-speaker model (n_speakers == 0).  Honours "length_aware". */
+size_t wetts_vits_voice_conversion_workspace_bytes(wetts_vits_t h, int B, int T);
+int wetts_vits_voice_conversion(wetts_vits_t h, const float* y, const int64_t* y_lengths, const int64_t* sid_src,
+                                const int64_t* sid_tgt, const float* noise, int B, int T, float* audio, float* y_mask,
+                                float* z, float* z_p, float* z_hat, void* workspace, size_t workspace_bytes,
                                 void* stream);
 
 /* ---- L2 session contract (export_onnx.py:93-148; VitsModel::ForwardDecoder) --

@@ -52,6 +52,7 @@ PROTOTYPES = {
     "wetts_expand_prior": (_I, [_P, _P, _P, _P, _P, _P, _P, _I64, _I64, _F, _I, _I, _I, _P, _P, _P, _P, _P, _P]),
     "wetts_flow_workspace_bytes": (_SZ, [_P, _I, _I]),
     "wetts_flow_reverse": (_I, [_P, _P, _P, _P, _I, _I, _P, _SZ, _P]),
+    "wetts_flow_forward": (_I, [_P, _P, _P, _P, _I, _I, _P, _SZ, _P]),
     "wetts_generator_workspace_bytes": (_SZ, [_P, _I, _I]),
     "wetts_generator_forward": (_I, [_P, _P, _P, _P, _I, _I, _P, _P, _SZ, _P]),
     "wetts_generator_forward_view": (_I, [_P, _P, _I64, _I64, _P, _P, _I, _I, _P, _P, _SZ, _P]),
@@ -61,6 +62,12 @@ PROTOTYPES = {
                                          _SZ, _P]),
     "wetts_vits_decoder_workspace_bytes": (_SZ, [_P, _I, _I]),
     "wetts_vits_forward_decoder": (_I, [_P, _P, _P, _I, _I, _P, _P, _SZ, _P]),
+    "wetts_posterior_workspace_bytes": (_SZ, [_P, _I, _I]),
+    "wetts_posterior_encoder_forward": (_I, [_P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _SZ, _P]),
+    "wetts_spectrogram_workspace_bytes": (_SZ, [_P, _I, _I64]),
+    "wetts_spectrogram": (_I, [_P, _P, _P, _I, _I64, _P, _P, _P, _SZ, _P]),
+    "wetts_vits_voice_conversion_workspace_bytes": (_SZ, [_P, _I, _I]),
+    "wetts_vits_voice_conversion": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "wetts_audio_to_int16": (_I, [_P, _P, _I, _I64, _I, _P, _P, _P]),
     "wetts_vits_check_fault": (_I, [_P, _P, _I]),
     "wetts_vits_launch_count": (C.c_uint64, [_P]),

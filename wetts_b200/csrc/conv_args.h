@@ -12,7 +12,7 @@ enum EpiMode : int {
   EPI_MRF = 2,       // val = v + resid; acc_mode 0: out=val, 1: out+=val, 2: out=(out+val)/div
   EPI_GATE = 3,      // paired channels -> tanh(a+ga)*sigmoid(b+gb)   (modules.py:76-77)
   EPI_RES_SKIP = 4,  // co<H: x=(x+v)*mask ; co>=H: skip(+)=v         (modules.py:81-86)
-  EPI_COUPLING = 5,  // z1 = (z1 - v*mask)*mask                       (flows.py:510)
+  EPI_COUPLING = 5,  // z1 = (z1 - v*mask)*mask  (flows.py:510); z_forward: z1 = (z1 + v*mask)*mask  (flows.py:505)
   EPI_CONVT = 6,     // polyphase ConvTranspose1d scatter (tensor-core path only)
 };
 
@@ -35,6 +35,7 @@ struct ConvEpilogue {
   int last = 0;              // last WN layer: all Cout channels go to skip
   int z_c0 = 0;              // EPI_COUPLING: target channel = z_c0 + co*z_cstep in `out`
   int z_cstep = 1;
+  int z_forward = 0;         // EPI_COUPLING: 0 = inverse direction (subtract the mean), 1 = forward (add it)
   int up_u = 1, up_pad = 0;  // EPI_CONVT: stride and padding of the transposed conv
   long long out_T = 0;       // EPI_CONVT: output samples per channel
 };

@@ -180,6 +180,17 @@ struct wetts_vits_s {
     bool flipped = false;
     PlainEncLayer tf[2];   // flow_type 1 only
   } flow[4];  // application order: reference layers 6, 4, 2, 0
+  // posterior encoder (enc_q, models.py:124-132; encoders.py:60-99): packed only when the checkpoint carries every key
+  static constexpr int kPostLayers = 16;
+  struct Posterior {
+    Conv pre, cond, proj, in[kPostLayers], rs[kPostLayers];
+    int S = 0;   // feature channels of enc_q.pre: filter_length / 2 + 1 (linear spectrogram) or n_mel_channels
+  } post;
+  bool has_post = false;
+  std::string post_missing;   // first missing enc_q key when !has_post
+  // linear spectrogram (mel_processing.py:42-93 with center=False): windowed real DFT as a constant 1x1 conv
+  Conv spec_dft;
+  int spec_nfft = 0;   // 0: the feature dimension is not n_fft/2 + 1 of a power-of-two n_fft (no spectrogram)
   // Vocos generator (vocoder_type 1)
   struct ConvNext {
     float *dww = nullptr, *dwb = nullptr;
@@ -407,6 +418,24 @@ static void run_dds(const Dds& d, float* x, float* y, float* y2, const long long
   }
 }
 
+// WN (modules.py:60-87) on the gated / res-skip epilogues: x [B][H][T] is the residual stream (updated in place and
+// masked), skip [B][H][T] receives the unmasked sum of the skip outputs (the caller masks it through the next conv's
+// in_mask).  gc: per-utterance cond vectors [B][2*H*n_layers] of the layer's cond_layer, or nullptr.
+static void run_wn(const Conv* in, const Conv* rs, int n_layers, float* x, float* acts, float* skip, const float* gc,
+                   const long long* len, int B, int H, int T, cudaStream_t s) {
+  for (int i = 0; i < n_layers; ++i) {
+    ConvArgs a = conv_args(in[i], x, (long long)H * T, T, B, T);
+    a.ep.mode = EPI_GATE; a.ep.H = H; a.ep.out = acts; a.ep.out_bs = (long long)H * T;
+    if (gc) { a.ep.cond = gc; a.ep.cond_bs = 2 * H * n_layers; a.ep.cond_off = 2 * H * i; }
+    launch_conv1d(a, s);
+    a = conv_args(rs[i], acts, (long long)H * T, T, B, T);
+    a.lengths = len;
+    a.ep.mode = EPI_RES_SKIP; a.ep.H = H; a.ep.x = x; a.ep.skip = skip; a.ep.out_bs = (long long)H * T;
+    a.ep.skip_init = (i == 0); a.ep.last = (i == n_layers - 1);
+    launch_conv1d(a, s);
+  }
+}
+
 }  // namespace wetts
 
 // ================================================================== C ABI
@@ -578,7 +607,6 @@ uint64_t wetts_vits_launch_count(wetts_vits_t h) { return h ? kernel_launch_coun
 int wetts_vits_set_tensor(wetts_vits_t h, const char* name, const void* data, const int64_t* dims, int ndim) {
   if (!h || !name || !data || (!dims && ndim > 0)) return fail("null argument");
   if (h->finalized) return fail("handle is finalized (immutable)");
-  if (!strncmp(name, "enc_q.", 6)) return 0;  // posterior encoder: never on the inference path
   CUDA_OK(cudaSetDevice(h->device));
   Raw r;
   r.dims.assign(dims, dims + ndim);
@@ -902,6 +930,49 @@ int wetts_vits_finalize(wetts_vits_t h) {
     if (r->dims.size() != 3 || r->dims[0] != 1 || r->dims[1] != ch) return fail("dec.conv_post.weight: unexpected shape");
     h->conv_post_w = r->d;
   }
+  // ---- posterior encoder (voice conversion only; infer never reads it)
+  {
+    const int nl = wetts_vits_s::kPostLayers;
+    auto has_conv = [&](const std::string& p) { return h->find(p + ".weight") || (h->find(p + ".weight_g") && h->find(p + ".weight_v")); };
+    std::vector<std::string> convs = {"enc_q.pre"};
+    for (int i = 0; i < nl; ++i) convs.push_back("enc_q.enc.in_layers." + std::to_string(i));
+    for (int i = 0; i < nl; ++i) convs.push_back("enc_q.enc.res_skip_layers." + std::to_string(i));
+    if (gin) convs.push_back("enc_q.enc.cond_layer");
+    convs.push_back("enc_q.proj");
+    for (const auto& p : convs) {
+      if (!has_conv(p)) { h->post_missing = p + (h->find(p + ".weight_g") ? ".weight_v" : h->find(p + ".weight_v") ? ".weight_g" : ".weight"); break; }
+      if (!h->find(p + ".bias")) { h->post_missing = p + ".bias"; break; }
+    }
+    if (h->post_missing.empty()) {
+      auto& P = h->post;
+      std::vector<int> gate(2 * H);
+      for (int q = 0; q < 2 * H; ++q) gate[q] = (q & 1) ? H + (q >> 1) : (q >> 1);
+      if (h->make_conv("enc_q.pre", &P.pre)) return 1;
+      if (P.pre.K != 1 || P.pre.Cout != H) return fail("enc_q.pre: expected a 1x1 conv to %d channels", H);
+      P.S = P.pre.Cin;
+      if (gin && h->make_conv("enc_q.enc.cond_layer", &P.cond)) return 1;
+      if (gin && P.cond.Cout != 2 * H * nl) return fail("enc_q.enc.cond_layer: expected %d output channels", 2 * H * nl);
+      for (int i = 0; i < nl; ++i) {
+        if (h->make_conv("enc_q.enc.in_layers." + std::to_string(i), &P.in[i], true, gate)) return 1;
+        if (P.in[i].K != 5 || P.in[i].Cin != H) return fail("enc_q.enc.in_layers.%d: expected [%d,%d,5]", i, 2 * H, H);
+        if (h->make_conv("enc_q.enc.res_skip_layers." + std::to_string(i), &P.rs[i])) return 1;
+        if (P.rs[i].Cout != (i < nl - 1 ? 2 * H : H)) return fail("enc_q.enc.res_skip_layers.%d: unexpected shape", i);
+      }
+      if (h->make_conv("enc_q.proj", &P.proj)) return 1;
+      if (P.proj.K != 1 || P.proj.Cout != 2 * Cc || P.proj.Cin != H) return fail("enc_q.proj: expected [%d,%d,1]", 2 * Cc, H);
+      h->has_post = true;
+      // linear spectrogram front end: n_fft = 2 (S - 1) for a power-of-two n_fft, hop = the upsample factor
+      const int N = 2 * (P.S - 1);
+      if (P.S >= 9 && !((P.S - 1) & (P.S - 2)) && h->U <= N && (N - h->U) % 2 == 0) {
+        Raw wd;
+        wd.dims = {(int64_t)N + 2, (int64_t)N, 1};
+        if (h->dalloc(&wd.d, wd.numel())) return 1;
+        launch_dft_weight(wd.d, N, 0);
+        if (h->pack_conv_from(wd, nullptr, {}, {}, &h->spec_dft)) return 1;
+        h->spec_nfft = N;
+      }
+    }
+  }
   if (c.n_speakers > 0) {
     if (h->need("emb_g.weight", &r)) return 1;
     if (r->dims.size() != 2 || r->dims[0] != c.n_speakers || r->dims[1] != gin) return fail("emb_g.weight: unexpected shape");
@@ -1178,11 +1249,14 @@ size_t wetts_flow_workspace_bytes(wetts_vits_t h, int B, int Ty) {
   FlowWs w;
   return flow_layout(h->cfg, B, Ty, A, &w) + 256;
 }
-int wetts_flow_reverse(wetts_vits_t h, float* z, const int64_t* y_lengths, const float* g, int B, int Ty, void* workspace,
-                       size_t workspace_bytes, void* stream) {
-  CHECK_READY(h);
+}  // extern "C"
+
+// The four coupling layers of the flow.  Inverse (infer): reference layers 6, 4, 2, 0, each x1 = (x1 - m) * mask.
+// Forward (voice conversion): layers 0, 2, 4, 6, each x1 = m + x1 * mask (flows.py:494-513, mean_only).  The Flips between
+// them are folded into channel maps; a layer sees z reversed (`flipped`) in both directions alike.
+static int flow_run(wetts_vits_t h, float* z, const int64_t* y_lengths, const float* g, int B, int Ty, void* workspace,
+                    size_t workspace_bytes, cudaStream_t s, bool forward) {
   const wetts_vits_config& c = h->cfg;
-  cudaStream_t s = (cudaStream_t)stream;
   Arena A(workspace, workspace_bytes);
   FlowWs w;
   flow_layout(c, B, Ty, A, &w);
@@ -1190,8 +1264,8 @@ int wetts_flow_reverse(wetts_vits_t h, float* z, const int64_t* y_lengths, const
   const int H = c.hidden_channels, Cc = c.inter_channels, half = Cc / 2;
   const long long* len = (const long long*)y_lengths;
   const bool has_g = g && c.gin_channels > 0;
-  for (int j = 0; j < 4; ++j) {
-    auto& F = h->flow[j];
+  for (int step = 0; step < 4; ++step) {
+    auto& F = h->flow[forward ? 3 - step : step];
     if (has_g) cond_vector(F.cond, g, B, w.gc, s);
     ConvArgs a;
     if (c.flow_type == 1) {
@@ -1230,27 +1304,30 @@ int wetts_flow_reverse(wetts_vits_t h, float* z, const int64_t* y_lengths, const
     }
     a.lengths = len; a.ep.out_mask = 1; a.ep.out = w.hb;
     launch_conv1d(a, s);
-    for (int i = 0; i < 4; ++i) {
-      a = conv_args(F.in[i], w.hb, (long long)H * Ty, Ty, B, Ty);
-      a.ep.mode = EPI_GATE; a.ep.H = H; a.ep.out = w.acts; a.ep.out_bs = (long long)H * Ty;
-      if (has_g) { a.ep.cond = w.gc; a.ep.cond_bs = 8 * H; a.ep.cond_off = 2 * H * i; }
-      launch_conv1d(a, s);
-      a = conv_args(F.rs[i], w.acts, (long long)H * Ty, Ty, B, Ty);
-      a.lengths = len;
-      a.ep.mode = EPI_RES_SKIP; a.ep.H = H; a.ep.x = w.hb; a.ep.skip = w.skip; a.ep.out_bs = (long long)H * Ty;
-      a.ep.skip_init = (i == 0); a.ep.last = (i == 3);
-      launch_conv1d(a, s);
-    }
-    // m = post(out * mask) * mask ; x1 = (x1 - m) * mask
+    run_wn(F.in, F.rs, 4, w.hb, w.acts, w.skip, has_g ? w.gc : nullptr, len, B, H, Ty, s);
+    // m = post(out * mask) * mask ; x1 = (x1 - m) * mask  (forward: x1 = m + x1 * mask)
     a = conv_args(F.post, w.skip, (long long)H * Ty, Ty, B, Ty);
     a.lengths = len; a.in_mask = 1;
     a.ep.mode = EPI_COUPLING; a.ep.out = z; a.ep.out_bs = (long long)Cc * Ty;
     a.ep.z_c0 = F.flipped ? half - 1 : half;
     a.ep.z_cstep = F.flipped ? -1 : 1;
+    a.ep.z_forward = forward ? 1 : 0;
     launch_conv1d(a, s);
   }
   CHECK_LAUNCH();
   return 0;
+}
+
+extern "C" {
+int wetts_flow_reverse(wetts_vits_t h, float* z, const int64_t* y_lengths, const float* g, int B, int Ty, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  CHECK_READY(h);
+  return flow_run(h, z, y_lengths, g, B, Ty, workspace, workspace_bytes, (cudaStream_t)stream, false);
+}
+int wetts_flow_forward(wetts_vits_t h, float* z, const int64_t* y_lengths, const float* g, int B, int Ty, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  CHECK_READY(h);
+  return flow_run(h, z, y_lengths, g, B, Ty, workspace, workspace_bytes, (cudaStream_t)stream, true);
 }
 
 // ------------------------------------------------------------------ generator
@@ -1593,6 +1670,182 @@ int wetts_vits_infer_synthesize(wetts_vits_t h, const int64_t* x_lengths, const 
                                    w.scratch_bytes, stream))
     return 1;
   return 0;
+}
+
+// ------------------------------------------------------------------ voice conversion (models.py:369-376)
+#define CHECK_POSTERIOR(h)                                                                                      \
+  if (!(h)->has_post)                                                                                           \
+    return fail("the checkpoint has no complete posterior encoder: missing checkpoint tensor '%s'", (h)->post_missing.c_str());
+
+struct PostWs {
+  float *gc, *hb, *acts, *skip, *stats;
+};
+static size_t post_layout(const wetts_vits_config& c, int B, int T, Arena& A, PostWs* w) {
+  const size_t H = c.hidden_channels, n = (size_t)B * T;
+  w->gc = A.take<float>((size_t)B * 2 * H * wetts_vits_s::kPostLayers);
+  w->hb = A.take<float>(H * n);
+  w->acts = A.take<float>(H * n);
+  w->skip = A.take<float>(H * n);
+  w->stats = A.take<float>((size_t)2 * c.inter_channels * n);
+  return A.off;
+}
+size_t wetts_posterior_workspace_bytes(wetts_vits_t h, int B, int T) {
+  if (!h) return 0;
+  Arena A(nullptr, 0);
+  PostWs w;
+  return post_layout(h->cfg, B, T, A, &w) + 256;
+}
+// PosteriorEncoder.forward (encoders.py:91-99): pre(y) * mask, WN(16 layers, g), proj(.) * mask, z = (m + noise*exp(logs)) * mask
+static int posterior_run(wetts_vits_t h, const float* y, const int64_t* y_lengths, const float* g, const float* noise, int B,
+                         int T, float* z, float* m, float* logs, float* y_mask, void* workspace, size_t workspace_bytes,
+                         cudaStream_t s) {
+  CHECK_POSTERIOR(h);
+  if (!y || !y_lengths || !noise || !z) return fail("null argument");
+  if (B <= 0 || T <= 0) return fail("empty batch");
+  const wetts_vits_config& c = h->cfg;
+  Arena A(workspace, workspace_bytes);
+  PostWs w;
+  post_layout(c, B, T, A, &w);
+  if (!workspace || !A.ok()) return fail("posterior encoder workspace too small: need %zu bytes", A.off);
+  const auto& P = h->post;
+  const int H = c.hidden_channels;
+  const long long* len = (const long long*)y_lengths;
+  const bool has_g = g && c.gin_channels > 0;
+  ConvArgs a = conv_args(P.pre, y, (long long)P.S * T, T, B, T);
+  a.lengths = len; a.ep.out_mask = 1; a.ep.out = w.hb;
+  launch_conv1d(a, s);
+  if (has_g) cond_vector(P.cond, g, B, w.gc, s);
+  run_wn(P.in, P.rs, wetts_vits_s::kPostLayers, w.hb, w.acts, w.skip, has_g ? w.gc : nullptr, len, B, H, T, s);
+  a = conv_args(P.proj, w.skip, (long long)H * T, T, B, T);
+  a.lengths = len; a.in_mask = 1; a.ep.out_mask = 1; a.ep.out = w.stats;
+  launch_conv1d(a, s);
+  launch_posterior_sample(w.stats, noise, len, z, m, logs, y_mask, B, c.inter_channels, T, s);
+  CHECK_LAUNCH();
+  return 0;
+}
+int wetts_posterior_encoder_forward(wetts_vits_t h, const float* y, const int64_t* y_lengths, const float* g, const float* noise,
+                                    int B, int T, float* z, float* m, float* logs, void* workspace, size_t workspace_bytes,
+                                    void* stream) {
+  CHECK_READY(h);
+  return posterior_run(h, y, y_lengths, g, noise, B, T, z, m, logs, nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ---- linear spectrogram (spectrogram_torch, mel_processing.py:42-93, center=False, per utterance)
+struct SpecGeom {
+  int N, K, hop, pad, F;
+};
+static int spec_geometry(wetts_vits_t h, int64_t L, SpecGeom* g) {
+  CHECK_POSTERIOR(h);
+  if (!h->spec_nfft)
+    return fail("the posterior encoder takes %d feature channels, not n_fft/2+1 of a power-of-two n_fft: there is no linear "
+                "spectrogram for it (a mel posterior encoder takes the caller's mel features)", h->post.S);
+  g->N = h->spec_nfft;
+  g->K = g->N / 2 + 1;
+  g->hop = h->U;
+  g->pad = (g->N - g->hop) / 2;
+  if (L <= g->pad) return fail("audio of %lld samples is shorter than the %d + 1 the spectrogram's reflection padding needs",
+                               (long long)L, g->pad);
+  g->F = (int)(1 + (L + 2 * g->pad - g->N) / g->hop);
+  return 0;
+}
+static size_t spec_layout(const SpecGeom& sg, int B, Arena& A, float** frames, float** dft) {
+  *frames = A.take<float>((size_t)B * sg.N * sg.F);
+  *dft = A.take<float>((size_t)B * 2 * sg.K * sg.F);
+  return A.off;
+}
+size_t wetts_spectrogram_workspace_bytes(wetts_vits_t h, int B, int64_t L) {
+  if (!h) return 0;
+  SpecGeom sg;
+  if (spec_geometry(h, L, &sg)) return 0;
+  Arena A(nullptr, 0);
+  float *f, *d;
+  return spec_layout(sg, B, A, &f, &d) + 256;
+}
+int wetts_spectrogram(wetts_vits_t h, const float* audio, const int64_t* audio_lengths, int B, int64_t L, float* spec,
+                      int64_t* spec_lengths, void* workspace, size_t workspace_bytes, void* stream) {
+  CHECK_READY(h);
+  if (!audio || !audio_lengths || !spec) return fail("null argument");
+  if (B <= 0) return fail("empty batch");
+  SpecGeom sg;
+  if (spec_geometry(h, L, &sg)) return 1;
+  cudaStream_t s = (cudaStream_t)stream;
+  Arena A(workspace, workspace_bytes);
+  float *frames, *dft;
+  spec_layout(sg, B, A, &frames, &dft);
+  if (!workspace || !A.ok()) return fail("spectrogram workspace too small: need %zu bytes", A.off);
+  // every utterance must be longer than the reflection padding (torch's reflect pad rejects it otherwise): the lengths
+  // are checked on the host, so this call synchronises `stream`
+  std::vector<long long> lens(B);
+  CUDA_OK(cudaMemcpyAsync(lens.data(), audio_lengths, sizeof(long long) * B, cudaMemcpyDeviceToHost, s));
+  CUDA_OK(cudaStreamSynchronize(s));
+  for (int b = 0; b < B; ++b)
+    if (lens[b] <= sg.pad || lens[b] > L)
+      return fail("utterance %d has %lld samples: need %d < length <= %lld (the reflection padding of the spectrogram)", b,
+                  lens[b], sg.pad, (long long)L);
+  const long long* len = (const long long*)audio_lengths;
+  launch_spec_frames(audio, (long long)L, len, frames, B, sg.N, sg.hop, sg.pad, sg.F, s);
+  ConvArgs a = conv_args(h->spec_dft, frames, (long long)sg.N * sg.F, sg.F, B, sg.F);
+  a.ep.out = dft;
+  launch_conv1d(a, s);
+  launch_spec_magnitude(dft, len, spec, (long long*)spec_lengths, B, sg.K, sg.F, sg.N, sg.hop, sg.pad, s);
+  CHECK_LAUNCH();
+  return 0;
+}
+
+// ---- the composite call: posterior encoder (g_src), forward flow (g_src), inverse flow (g_tgt), dec(z_hat * y_mask, g_tgt)
+struct VcWs {
+  float *g_src, *g_tgt, *z, *z_p, *z_hat;
+  void* scratch;
+  size_t scratch_bytes;
+};
+static size_t vc_layout(wetts_vits_t h, int B, int T, Arena& A, VcWs* w) {
+  const wetts_vits_config& c = h->cfg;
+  const size_t n = (size_t)B * c.inter_channels * T;
+  w->g_src = A.take<float>((size_t)B * (c.gin_channels > 0 ? c.gin_channels : 1));
+  w->g_tgt = A.take<float>((size_t)B * (c.gin_channels > 0 ? c.gin_channels : 1));
+  w->z = A.take<float>(n);
+  w->z_p = A.take<float>(n);
+  w->z_hat = A.take<float>(n);
+  size_t mx = wetts_posterior_workspace_bytes(h, B, T);
+  const size_t s2 = wetts_flow_workspace_bytes(h, B, T), s3 = wetts_generator_workspace_bytes(h, B, T);
+  mx = mx > s2 ? mx : s2;
+  mx = mx > s3 ? mx : s3;
+  w->scratch = A.take<char>(mx);
+  w->scratch_bytes = mx;
+  return A.off;
+}
+size_t wetts_vits_voice_conversion_workspace_bytes(wetts_vits_t h, int B, int T) {
+  if (!h) return 0;
+  Arena A(nullptr, 0);
+  VcWs w;
+  return vc_layout(h, B, T, A, &w) + 256;
+}
+int wetts_vits_voice_conversion(wetts_vits_t h, const float* y, const int64_t* y_lengths, const int64_t* sid_src,
+                                const int64_t* sid_tgt, const float* noise, int B, int T, float* audio, float* y_mask, float* z,
+                                float* z_p, float* z_hat, void* workspace, size_t workspace_bytes, void* stream) {
+  CHECK_READY(h);
+  CHECK_POSTERIOR(h);
+  if (h->cfg.n_speakers <= 0) return fail("voice conversion needs a multi-speaker model (n_speakers == 0)");
+  if (!y || !y_lengths || !sid_src || !sid_tgt || !noise || !audio) return fail("null argument");
+  if (B <= 0 || T <= 0) return fail("empty batch");
+  const wetts_vits_config& c = h->cfg;
+  cudaStream_t s = (cudaStream_t)stream;
+  Arena A(workspace, workspace_bytes);
+  VcWs w;
+  vc_layout(h, B, T, A, &w);
+  if (!workspace || !A.ok()) return fail("voice conversion workspace too small: need %zu bytes", A.off);
+  const size_t zbytes = sizeof(float) * (size_t)B * c.inter_channels * T;
+  float* zb = z ? z : w.z;
+  float* zpb = z_p ? z_p : w.z_p;
+  float* zhb = z_hat ? z_hat : w.z_hat;
+  if (wetts_speaker_embedding(h, sid_src, B, w.g_src, stream) || wetts_speaker_embedding(h, sid_tgt, B, w.g_tgt, stream)) return 1;
+  if (posterior_run(h, y, y_lengths, w.g_src, noise, B, T, zb, nullptr, nullptr, y_mask, w.scratch, w.scratch_bytes, s)) return 1;
+  CUDA_OK(cudaMemcpyAsync(zpb, zb, zbytes, cudaMemcpyDeviceToDevice, s));
+  if (wetts_flow_forward(h, zpb, y_lengths, w.g_src, B, T, w.scratch, w.scratch_bytes, stream)) return 1;
+  CUDA_OK(cudaMemcpyAsync(zhb, zpb, zbytes, cudaMemcpyDeviceToDevice, s));
+  if (wetts_flow_reverse(h, zhb, y_lengths, w.g_tgt, B, T, w.scratch, w.scratch_bytes, stream)) return 1;
+  // models.py:376: the vocoder sees z_hat * y_mask over the full padded length
+  return wetts_generator_forward(h, zhb, y_lengths, w.g_tgt, B, T, audio, w.scratch, w.scratch_bytes, stream);
 }
 
 // ------------------------------------------------------------------ L2 decoder contract

@@ -91,6 +91,7 @@ __device__ __forceinline__ void epilogue_finish(const ConvArgs& a, int b, int co
     }
     case EPI_COUPLING: {
       const int zc = e.z_c0 + co * e.z_cstep;
+      if (e.z_forward) v = -v;   // exact: the inverse direction keeps its expression (and its FMA) bit for bit
       e.out[(long long)b * e.out_bs + (long long)zc * T + t] = (l.a - v * msk) * msk;
       break;
     }

@@ -168,6 +168,18 @@ void launch_istft_overlap_add(const float* frames /*[B][N][F]*/, float* out /*[B
 void launch_scale_rows(const float* w, const float* bias, const float* sc, float* w_out, float* b_out, int rows, int cols,
                        cudaStream_t s);
 
+// ---------------------------------------------------------------- posterior encoder / linear spectrogram (voice conversion)
+// stats [B][2C][T] -> z = (m + noise * exp(logs)) * mask; m, logs [B][C][T] and y_mask [B][1][T] optional
+void launch_posterior_sample(const float* stats, const float* noise, const long long* lengths, float* z, float* m, float* logs,
+                             float* y_mask, int B, int C, int T, cudaStream_t s);
+// audio [B][L] -> frames [B][N][F] of each utterance reflect-padded by `pad` at its own length (0 beyond its F_b frames)
+void launch_spec_frames(const float* audio, long long L, const long long* lengths, float* frames, int B, int N, int hop, int pad,
+                        int F, cudaStream_t s);
+void launch_dft_weight(float* w /*[N+2][N][1]*/, int N, cudaStream_t s);
+// dft [B][2K][F] -> spec [B][K][F] magnitudes (+1e-6 inside the root), 0 beyond F_b; spec_lengths int64[B] (optional)
+void launch_spec_magnitude(const float* dft, const long long* lengths, float* spec, long long* spec_lengths, int B, int K, int F,
+                           int N, int hop, int pad, cudaStream_t s);
+
 unsigned long long kernel_launch_counter();
 void count_launch();
 

@@ -402,6 +402,71 @@ __global__ void istft_overlap_add_kernel(const float* __restrict__ frames, float
   }
   out[(long long)b * L + t] = acc / env;
 }
+// ------------------------------------------------------------------ posterior encoder / linear spectrogram
+// stats [B][2C][T] (m rows 0..C-1, logs rows C..2C-1, already masked) -> z = (m + noise * exp(logs)) * mask
+// (encoders.py:97-98); m / logs / y_mask written when non-null (y_mask [B][1][T] by the c == 0 threads)
+__global__ void posterior_sample_kernel(const float* __restrict__ stats, const float* __restrict__ noise,
+                                        const long long* __restrict__ lengths, float* __restrict__ z, float* __restrict__ m_out,
+                                        float* __restrict__ logs_out, float* __restrict__ y_mask, int C, int T) {
+  const int b = blockIdx.z, c = blockIdx.y, t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= T) return;
+  const float msk = t < lengths[b] ? 1.f : 0.f;
+  const long long o = ((long long)b * C + c) * T + t;
+  const float m = stats[((long long)b * 2 * C + c) * T + t];
+  const float ls = stats[((long long)b * 2 * C + C + c) * T + t];
+  z[o] = (m + noise[o] * expf(ls)) * msk;
+  if (m_out) m_out[o] = m;
+  if (logs_out) logs_out[o] = ls;
+  if (y_mask && c == 0) y_mask[(long long)b * T + t] = msk;
+}
+// frames[b][n][f] = audio[b][reflect(f*hop + n - pad)] for f < F_b (the frames torch.stft(center=False) takes from the
+// utterance reflect-padded by `pad` at its own length L_b), 0 for f >= F_b.  The analysis window is in the DFT weight.
+__global__ void spec_frames_kernel(const float* __restrict__ audio, long long L, const long long* __restrict__ lengths,
+                                   float* __restrict__ frames, int N, int hop, int pad, int F) {
+  const int b = blockIdx.z, n = blockIdx.y, f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= F) return;
+  const long long Lb = lengths[b];
+  const long long Fb = 1 + (Lb + 2 * pad - N) / hop;
+  float v = 0.f;
+  if (f < Fb) {
+    long long i = (long long)f * hop + n - pad;
+    if (i < 0) i = -i;
+    if (i >= Lb) i = 2 * (Lb - 1) - i;
+    v = audio[(long long)b * L + i];
+  }
+  frames[((long long)b * N + n) * F + f] = v;
+}
+// forward real DFT x periodic hann window as a 1x1 conv weight [2K][N][1] (K = N/2 + 1): row k = re, row K + k = im
+// (the forward twin of idft_weight_kernel)
+__global__ void dft_weight_kernel(float* __restrict__ w, int N) {
+  const int K = N / 2 + 1;
+  const long long total = (long long)2 * K * N;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int n = (int)(i % N), row = (int)(i / N);
+    const int k = row < K ? row : row - K;
+    const long long kn = ((long long)k * n) % N;                       // exact angle reduction
+    const double ang = 6.283185307179586476925286766559 * (double)kn / (double)N;
+    const double win = 0.5 - 0.5 * cos(6.283185307179586476925286766559 * (double)n / (double)N);   // periodic hann
+    w[i] = (float)((row < K ? cos(ang) : -sin(ang)) * win);
+  }
+}
+// dft [B][2K][F] (re | im) -> spec [B][K][F] = sqrt(re^2 + im^2 + 1e-6) for f < F_b, exactly 0 beyond
+// (mel_processing.py:91); spec_lengths[b] = F_b written by the (k == 0, f == 0) thread
+__global__ void spec_magnitude_kernel(const float* __restrict__ dft, const long long* __restrict__ lengths, float* __restrict__ spec,
+                                      long long* __restrict__ spec_lengths, int K, int F, int N, int hop, int pad) {
+  const int b = blockIdx.z, k = blockIdx.y, f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= F) return;
+  const long long Fb = 1 + (lengths[b] + 2 * pad - N) / hop;
+  float v = 0.f;
+  if (f < Fb) {
+    const float re = dft[((long long)b * 2 * K + k) * F + f];
+    const float im = dft[((long long)b * 2 * K + K + k) * F + f];
+    v = sqrtf(re * re + im * im + 1e-6f);
+  }
+  spec[((long long)b * K + k) * F + f] = v;
+  if (spec_lengths && k == 0 && f == 0) spec_lengths[b] = Fb;
+}
+
 // w[r][*] *= s[r], b[r] *= s[r]   (ConvNeXt layer scale folded into pw_conv2, decoders.py:245)
 __global__ void scale_rows_kernel(const float* __restrict__ w, const float* __restrict__ bias, const float* __restrict__ s,
                                   float* __restrict__ w_out, float* __restrict__ b_out, int rows, int cols) {
@@ -826,6 +891,29 @@ void launch_istft_overlap_add(const float* frames, float* out, int B, int N, int
 void launch_scale_rows(const float* w, const float* bias, const float* sc, float* w_out, float* b_out, int rows, int cols,
                        cudaStream_t s) {
   scale_rows_kernel<<<256, 256, 0, s>>>(w, bias, sc, w_out, b_out, rows, cols);
+  count_launch();
+}
+
+void launch_posterior_sample(const float* stats, const float* noise, const long long* lengths, float* z, float* m, float* logs,
+                             float* y_mask, int B, int C, int T, cudaStream_t s) {
+  dim3 grid((T + 127) / 128, C, B);
+  posterior_sample_kernel<<<grid, 128, 0, s>>>(stats, noise, lengths, z, m, logs, y_mask, C, T);
+  count_launch();
+}
+void launch_spec_frames(const float* audio, long long L, const long long* lengths, float* frames, int B, int N, int hop, int pad,
+                        int F, cudaStream_t s) {
+  dim3 grid((F + 127) / 128, N, B);
+  spec_frames_kernel<<<grid, 128, 0, s>>>(audio, L, lengths, frames, N, hop, pad, F);
+  count_launch();
+}
+void launch_dft_weight(float* w, int N, cudaStream_t s) {
+  dft_weight_kernel<<<1024, 256, 0, s>>>(w, N);
+  count_launch();
+}
+void launch_spec_magnitude(const float* dft, const long long* lengths, float* spec, long long* spec_lengths, int B, int K, int F,
+                           int N, int hop, int pad, cudaStream_t s) {
+  dim3 grid((F + 127) / 128, K, B);
+  spec_magnitude_kernel<<<grid, 128, 0, s>>>(dft, lengths, spec, spec_lengths, K, F, N, hop, pad);
   count_launch();
 }
 

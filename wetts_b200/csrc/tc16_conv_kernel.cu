@@ -176,8 +176,9 @@ __device__ __forceinline__ void tc16_epilogue_slice(const ConvArgs& a, int b, in
       float* zp = e.out + row + (size_t)(e.z_c0 + co0 * e.z_cstep) * Ts;
       const long long zstep = (long long)e.z_cstep * (long long)Ts;
       ld_strided<16>(zp, zstep, nval, r);
+      const float zsgn = e.z_forward ? -1.f : 1.f;   // forward direction: v * -1 (exact); inverse: v * 1 == v bit for bit
 #pragma unroll
-      for (int i = 0; i < 16; ++i) x[i] = (r[i] - v[i] * msk) * msk;
+      for (int i = 0; i < 16; ++i) x[i] = (r[i] - (v[i] * zsgn) * msk) * msk;
       st_strided<16>(zp, zstep, nval, x);
       break;
     }
@@ -269,8 +270,9 @@ __device__ __forceinline__ void tc16_epilogue_slice_r(const ConvArgs& a, int b, 
       break;
     }
     case EPI_COUPLING: {
+      const float zsgn = e.z_forward ? -1.f : 1.f;   // forward direction: v * -1 (exact); inverse: v * 1 == v bit for bit
 #pragma unroll
-      for (int i = 0; i < 16; ++i) x[i] = (r[i] - v[i] * msk) * msk;
+      for (int i = 0; i < 16; ++i) x[i] = (r[i] - (v[i] * zsgn) * msk) * msk;
       st_strided<16>(e.out + row + (size_t)(e.z_c0 + co0 * e.z_cstep) * Ts, (long long)e.z_cstep * (long long)Ts, nval, x);
       break;
     }

@@ -151,11 +151,12 @@ __device__ __forceinline__ void tc_epilogue_slice(const ConvArgs& a, int b, int 
       float* zp = e.out + row + (size_t)(e.z_c0 + co0 * e.z_cstep) * Ts;
       const long long step = (long long)e.z_cstep * (long long)Ts;
       float r[16];
+      const float zsgn = e.z_forward ? -1.f : 1.f;   // forward direction: v * -1 (exact); inverse: v * 1 == v bit for bit
 #pragma unroll
       for (int i = 0; i < 16; ++i) r[i] = (i < nval) ? zp[(long long)i * step] : 0.f;
 #pragma unroll
       for (int i = 0; i < 16; ++i)
-        if (i < nval) zp[(long long)i * step] = (r[i] - v[i] * msk) * msk;
+        if (i < nval) zp[(long long)i * step] = (r[i] - (v[i] * zsgn) * msk) * msk;
       break;
     }
     default:

@@ -173,8 +173,9 @@ WETTS_DEVICE void tc_epilogue_slice_m(const ConvArgs& a, int b, int t, int co0, 
       float* zp = e.out + row + (size_t)(e.z_c0 + co0 * e.z_cstep) * Ts;
       const long long zstep = (long long)e.z_cstep * (long long)Ts;
       ep_ld_strided<16>(zp, zstep, nval, r);
+      const float zsgn = e.z_forward ? -1.f : 1.f;   // forward direction: v * -1 (exact); inverse: v * 1 == v bit for bit
 #pragma unroll
-      for (int i = 0; i < 16; ++i) x[i] = (r[i] - v[i] * msk) * msk;
+      for (int i = 0; i < 16; ++i) x[i] = (r[i] - (v[i] * zsgn) * msk) * msk;
       ep_st_strided<16>(zp, zstep, nval, x);
       break;
     }

@@ -11,6 +11,8 @@ Additions over the reference signature (all keyword-only, default = reference be
 `noise_w` [B,2,Tx] and `noise_z` [B,192,>=Ty] inject the standard-normal draws the
 reference takes implicitly (duration_predictors.py:257, models.py:267), `durations`
 [B,1,Tx] teacher-forces ceil(w) for staged parity (SURVEY.md §0 findings 7-8).
+Likewise `voice_conversion(..., noise=)` / `enc_q(..., noise=)` take the posterior encoder's
+randn_like draw [B,192,T] (encoders.py:98).
 """
 import ctypes as C
 
@@ -88,7 +90,7 @@ class _Engine:
 
     def set_state(self, sd):
         self.pending = {k: v.detach().to(torch.float32).contiguous() for k, v in sd.items()
-                        if not k.startswith("enc_q.") and torch.is_tensor(v) and v.is_floating_point()}
+                        if torch.is_tensor(v) and v.is_floating_point()}
         if self.handle is not None:
             dev = self.device
             self.close()
@@ -200,22 +202,44 @@ class DurationPredictorBlock(_Block):
 
 
 class ResidualCouplingTransformersBlock(_Block):
-    """flows.py:442-449: forward(x, x_mask, g=None, reverse=False); inference (reverse=True) only."""
+    """flows.py:442-449: forward(x, x_mask, g=None, reverse=False) -> x.  reverse=True is the direction infer() takes,
+    reverse=False the one voice_conversion() takes first (z -> z_p)."""
 
     def forward(self, x, x_mask, g=None, reverse=False):
         e = self._e
         e.ready()
-        if not reverse:
-            raise NotImplementedError("forward (training) direction of the flow is out of scope")
         z = _f32(x, e.device).clone()
         B, _, Ty = z.shape
         lengths = _lengths_from_mask(x_mask.to(e.device))
         gv = None if g is None else _f32(g.reshape(B, -1), e.device)
         nbytes = e.lib.wetts_flow_workspace_bytes(e.handle, B, Ty)
         ws = e.workspace(nbytes)
-        check(e.lib.wetts_flow_reverse(e.handle, _ptr(z), _ptr(lengths), _ptr(gv), B, Ty, _ptr(ws), ws.numel(),
-                                       _stream(e.device)))
+        fn = e.lib.wetts_flow_reverse if reverse else e.lib.wetts_flow_forward
+        check(fn(e.handle, _ptr(z), _ptr(lengths), _ptr(gv), B, Ty, _ptr(ws), ws.numel(), _stream(e.device)))
         return z
+
+
+class PosteriorEncoder(_Block):
+    """encoders.py:91-99: forward(x, x_lengths, g=None) -> (z, m, logs, x_mask).  x [B, spec_channels, T] features;
+    `noise`: optional explicit N(0,1) [B,inter_channels,T] (the reference's randn_like)."""
+
+    def forward(self, x, x_lengths, g=None, *, noise=None):
+        e = self._e
+        e.ready()
+        x, x_lengths = _f32(x, e.device), _i64(x_lengths, e.device)
+        B, S, T = x.shape
+        Cc = e.cfg.inter_channels
+        noise = torch.randn(B, Cc, T, device=e.device) if noise is None else _f32(noise, e.device)
+        if tuple(noise.shape) != (B, Cc, T):
+            raise ValueError(f"noise has shape {tuple(noise.shape)}, need {(B, Cc, T)}")
+        gv = None if g is None else _f32(g.reshape(B, -1), e.device)
+        z, m, logs = (torch.empty(B, Cc, T, device=e.device, dtype=torch.float32) for _ in range(3))
+        nbytes = e.lib.wetts_posterior_workspace_bytes(e.handle, B, T)
+        ws = e.workspace(nbytes)
+        check(e.lib.wetts_posterior_encoder_forward(e.handle, _ptr(x), _ptr(x_lengths), _ptr(gv), _ptr(noise), B, T, _ptr(z),
+                                                    _ptr(m), _ptr(logs), _ptr(ws), ws.numel(), _stream(e.device)))
+        x_mask = (torch.arange(T, device=e.device)[None, :] < x_lengths[:, None]).to(torch.float32)[:, None, :]
+        return z, m, logs, x_mask
 
 
 class Generator(_Block):
@@ -264,6 +288,7 @@ class SynthesizerTrn:
         self.upsample_rates, self.upsample_kernel_sizes = list(upsample_rates), list(upsample_kernel_sizes)
         self.upsample_initial_channel = upsample_initial_channel
         self.n_speakers, self.gin_channels, self.use_sdp = n_speakers, gin_channels, bool(use_sdp)
+        self.use_mel_posterior_encoder = bool(kwargs.get("use_mel_posterior_encoder", False))
 
         c = VitsConfig()
         c.n_vocab, c.n_speakers = n_vocab, n_speakers
@@ -297,6 +322,7 @@ class SynthesizerTrn:
         self.dp = DurationPredictorBlock(self._engine)
         self.flow = ResidualCouplingTransformersBlock(self._engine)
         self.dec = Generator(self._engine)
+        self.enc_q = PosteriorEncoder(self._engine)
         if n_speakers > 0:
             self.emb_g = SpeakerEmbedding(self._engine)
         self.training = False
@@ -319,7 +345,13 @@ class SynthesizerTrn:
 
     def load_state_dict(self, state_dict, strict=False):
         """Accepts the reference's state dict as saved by task.py:59-76 (weight_g/weight_v pairs)
-        or with weight-norm already removed (export_onnx.py:79-81)."""
+        or with weight-norm already removed (export_onnx.py:79-81).  The posterior encoder (enc_q.*) is loaded
+        when present; its input channels must equal spec_channels."""
+        for k in ("enc_q.pre.weight", "enc_q.pre.weight_v"):
+            w = state_dict.get(k)
+            if torch.is_tensor(w) and w.dim() == 3 and w.shape[1] != self.spec_channels:
+                raise ValueError(f"{k} takes {w.shape[1]} feature channels, the model was built with "
+                                 f"spec_channels={self.spec_channels}")
         self._engine.set_state(state_dict)
         return self
 
@@ -397,6 +429,63 @@ class SynthesizerTrn:
                                                 ws.numel(), st))
         self.last_y_lengths = y_lengths
         return o, attn, y_mask, (z, z_p, m_p, logs_p)
+
+    # -- voice conversion (models.py:369-376) ---------------------------------
+    @torch.no_grad()
+    def spectrogram(self, audio, audio_lengths):
+        """spectrogram_torch (mel_processing.py:42-93, center=False) of each utterance on its own: audio [B,L] (or
+        [B,1,L]) in [-1,1], audio_lengths int64[B] -> (spec [B,spec_channels,F], spec_lengths int64[B]) with
+        F = 1 + (L + 2p - n_fft) // hop, n_fft = 2 (spec_channels - 1), hop = the upsample factor, p = (n_fft - hop) / 2.
+        Frames beyond an utterance's own count are 0.  Synchronises the current stream."""
+        if self.use_mel_posterior_encoder:
+            raise NotImplementedError("the mel posterior encoder takes mel features: pass them to voice_conversion()")
+        e = self._engine
+        e.ready()
+        audio = _f32(audio, e.device)
+        audio = audio.reshape(audio.shape[0], -1)
+        lengths = _i64(audio_lengths, e.device)
+        B, L = audio.shape
+        n_fft, hop = 2 * (self.spec_channels - 1), e.upsample
+        pad = (n_fft - hop) // 2
+        if L <= pad:
+            raise ValueError(f"audio of {L} samples is shorter than the {pad} + 1 the reflection padding needs")
+        F = 1 + (L + 2 * pad - n_fft) // hop
+        spec = torch.empty(B, self.spec_channels, F, device=e.device, dtype=torch.float32)
+        spec_lengths = torch.empty(B, device=e.device, dtype=torch.int64)
+        nbytes = e.lib.wetts_spectrogram_workspace_bytes(e.handle, B, L)
+        ws = e.workspace(max(int(nbytes), 1))
+        check(e.lib.wetts_spectrogram(e.handle, _ptr(audio), _ptr(lengths), B, L, _ptr(spec), _ptr(spec_lengths), _ptr(ws),
+                                      ws.numel(), _stream(e.device)))
+        return spec, spec_lengths
+
+    @torch.no_grad()
+    def voice_conversion(self, y, y_lengths, sid_src, sid_tgt, *, noise=None):
+        """models.py:369-376: y [B, spec_channels, T] features (linear spectrogram, see spectrogram(), or mel features for
+        the mel posterior encoder), y_lengths int64[B] -> (o_hat [B,1,T*U], y_mask [B,1,T], (z, z_p, z_hat)).
+        `noise`: optional explicit N(0,1) [B,inter_channels,T], the posterior encoder's randn_like draw."""
+        e = self._engine
+        e.ready()
+        dev = e.device
+        y, y_lengths = _f32(y, dev), _i64(y_lengths, dev)
+        B, S, T = y.shape
+        if S != self.spec_channels:
+            raise ValueError(f"y has {S} feature channels, the posterior encoder takes {self.spec_channels}")
+        if self.n_speakers <= 0:
+            raise WettsError("voice conversion needs a multi-speaker model (n_speakers == 0)")
+        sid_src, sid_tgt = _i64(sid_src, dev), _i64(sid_tgt, dev)
+        Cc = self.inter_channels
+        noise = torch.randn(B, Cc, T, device=dev) if noise is None else _f32(noise, dev)
+        if tuple(noise.shape) != (B, Cc, T):
+            raise ValueError(f"noise has shape {tuple(noise.shape)}, need {(B, Cc, T)}")
+        o = torch.empty(B, 1, T * e.upsample, device=dev, dtype=torch.float32)
+        y_mask = torch.empty(B, 1, T, device=dev, dtype=torch.float32)
+        z, z_p, z_hat = (torch.empty(B, Cc, T, device=dev, dtype=torch.float32) for _ in range(3))
+        nbytes = e.lib.wetts_vits_voice_conversion_workspace_bytes(e.handle, B, T)
+        ws = e.workspace(nbytes)
+        check(e.lib.wetts_vits_voice_conversion(e.handle, _ptr(y), _ptr(y_lengths), _ptr(sid_src), _ptr(sid_tgt), _ptr(noise),
+                                                B, T, _ptr(o), _ptr(y_mask), _ptr(z), _ptr(z_p), _ptr(z_hat), _ptr(ws),
+                                                ws.numel(), _stream(dev)))
+        return o, y_mask, (z, z_p, z_hat)
 
     # -- ONNX-export-shaped entry points (models.py:333-363) ------------------
     def export_forward(self, x, x_lengths, scales, sid):

@@ -194,8 +194,41 @@ def state_dict_spec(hps_model, n_vocab, n_speakers):
     return spec
 
 
+def posterior_spec(hps_model, spec_channels):
+    """Ordered (key, shape, kind) list of the posterior encoder `enc_q.*` (models.py:124-132, encoders.py:60-89):
+    pre 1x1 conv from `spec_channels`, a 16-layer WN (kernel 5, dilation 1) with gin conditioning, proj to 2*inter."""
+    m = _model_dict(hps_model)
+    H, inter, gin = m["hidden_channels"], m["inter_channels"], m.get("gin_channels", 0)
+    spec = [("enc_q.pre.weight", (H, spec_channels, 1), "conv_w"), ("enc_q.pre.bias", (H,), "conv_b")]
+
+    def wn_conv(prefix, dim0, dim1, k):
+        spec.extend([(prefix + ".bias", (dim0,), "conv_b"), (prefix + ".weight_g", (dim0, 1, 1), "wn_g"),
+                     (prefix + ".weight_v", (dim0, dim1, k), "wn_v")])
+
+    for i in range(16):
+        wn_conv(f"enc_q.enc.in_layers.{i}", 2 * H, H, 5)
+    for i in range(16):
+        wn_conv(f"enc_q.enc.res_skip_layers.{i}", 2 * H if i < 15 else H, H, 1)
+    if gin:
+        wn_conv("enc_q.enc.cond_layer", 2 * H * 16, gin, 1)
+    # proj: m and logs; kept small ("out_small") so that exp(logs) stays moderate on random weights
+    spec.extend([("enc_q.proj.weight", (2 * inter, H, 1), "out_small"), ("enc_q.proj.bias", (2 * inter,), "conv_b")])
+    return spec
+
+
+def posterior_state_dict(hps_model, spec_channels, n_speakers, seed=4321):
+    """Seeded synthetic `enc_q.*` tensors (fp32, CPU) to add to a make_state_dict() checkpoint for voice conversion.
+    `n_speakers` only documents the intended checkpoint: the posterior encoder's shapes do not depend on it."""
+    del n_speakers
+    return _generate(posterior_spec(hps_model, spec_channels), seed)
+
+
 def make_state_dict(hps_model, n_vocab, n_speakers, seed=1234):
     """Seeded synthetic `{"key": tensor}` dict (fp32, CPU)."""
+    return _generate(state_dict_spec(hps_model, n_vocab, n_speakers), seed)
+
+
+def _generate(spec, seed):
     gen = torch.Generator(device="cpu")
     gen.manual_seed(seed)
     sd = {}
@@ -207,7 +240,7 @@ def make_state_dict(hps_model, n_vocab, n_speakers, seed=1234):
     def uniform(shape, bound):
         return (torch.rand(shape, generator=gen, dtype=torch.float32) * 2 - 1) * bound
 
-    for key, shape, kind in state_dict_spec(hps_model, n_vocab, n_speakers):
+    for key, shape, kind in spec:
         if kind == "emb":
             t = randn(shape) * shape[1] ** -0.5
         elif kind == "rel":
